@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- faces/sec of the RetinaFace mnet25 detect path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (u8 images -> conv0..SSH -> fused heads+decode -> NMS)
 over one batch of synthetic S-real input (SURVEY.md 8d: the golden photo letter-boxed to the
@@ -19,14 +19,22 @@ Printed JSON (rank 0, one line):
              that kernel launched K times on the library's stream, vs MEASURED_PEAKS.json.
   configs    the other BASELINE.json configurations measured in the same run (device-timed + end to end): batch 1 / 32,
              configs[2] INT8 batch 32, configs[3] 1280x896; at --gpus 8: configs[4] INT8 batch 32 per GPU + all-gather.
-Timing: every number is the MEDIAN over blocks of K steps, blocks repeated until >= 0.3 s of timed work (a 2 ms window
-is not a measurement); `steps` stays K.  At N > 1 every step -- device-timed and end to end -- includes the exchange of
-the detection records (rf_detect_batch_device_allgather / rf_submit_batch_allgather: fused into the NMS kernel, comm.cu).
+Timing: every number times exactly K steps, after W untimed warm-up steps of the same kind.  The default K = 4000 makes
+the headline window about 0.3 s (77 us per step on a B200 at its 1000 W limit) and every other window at least as long,
+except batch 1 (about 0.1 s); a much smaller K times a window of a few ms, which measures the clock and the scheduler as
+much as the kernels.  At N > 1 every step -- device-timed and end to
+end -- includes the exchange of the detection records (rf_detect_batch_device_allgather / rf_submit_batch_allgather:
+fused into the NMS kernel, comm.cu).
   cpu_baseline  the oracle (cv2.dnn FP32 forward of the same caffemodel through a generated prototxt +
              oracle/postproc.c) timed on the host cores on a bounded sample (rank 0, N=1 only).
 
 --impl reference runs only that CPU arm (the reference's own CPU path cannot be built here:
 BVLC Caffe / OpenCV C++ / TensorRT are absent -- DESIGN.md), on the same config/metric/unit.
+
+--dump-outputs DIR writes, after the timed steps of --workload, what its last device-timed step returned (rank 0; at N > 1
+the gathered records of every rank): DIR/faces.npy (float32 [images][max_faces][15], FaceDetectInfo rows), DIR/anchor_index.npy
+and DIR/counts.npy (float64 [images][max_faces] and [images]); entries past an image's count are 0 (-1 for the anchor index).
+The inputs depend only on the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -62,7 +70,6 @@ WORKLOADS = {
 }
 EXTRA_1GPU = ["mnet25_fp16_b1_448", "mnet25_fp16_b32_448", "mnet0517_int8_b32_448", "mnet25_fp16_b8_1280x896"]
 EXTRA_NGPU = ["mnet0517_int8_b32_448_per_gpu"]
-MIN_TIMED_S = 0.3
 DEFAULT_WORKLOAD = "mnet25_fp16_b8_448"
 SCORE_THR, NMS_THR = 0.9, 0.4  # main.cpp:43, RetinaFace.h:66
 
@@ -88,9 +95,27 @@ def make_batches(wl, count, rank):
     return out
 
 
+def dump_device_outputs(out_dir, dets_ptr, counts_ptr, rows, max_faces, device):
+    """Writes the records of one rf_detect_batch_device[_allgather] call (rows x max_faces rf_det of 64 bytes, rows int32
+    counts; complete in device memory) to out_dir as faces / anchor_index / counts .npy files."""
+    import torch
+
+    class DeviceArray:
+        def __init__(self, ptr, shape, typestr):
+            self.__cuda_array_interface__ = dict(shape=shape, typestr=typestr, data=(ptr, False), version=2)
+
+    rec = torch.as_tensor(DeviceArray(dets_ptr, (rows, max_faces, 64), "|u1"), device=device).cpu().numpy()
+    counts = torch.as_tensor(DeviceArray(counts_ptr, (rows,), "<i4"), device=device).cpu().numpy()
+    valid = np.arange(max_faces)[None, :] < counts[:, None]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "faces.npy"), np.where(valid[..., None], rec.view(np.float32)[..., :15], 0).astype(np.float32))
+    np.save(os.path.join(out_dir, "anchor_index.npy"), np.where(valid, rec.view(np.int32)[..., 15], -1).astype(np.float64))
+    np.save(os.path.join(out_dir, "counts.npy"), counts.astype(np.float64))
+
+
 class ClockSampler(threading.Thread):
     """SM clock + throttle reasons sampled DURING the timed region: NVML every 2 ms when pynvml can open the device (the
-    timed region of the default run is ~30 ms), else one `nvidia-smi` query per 100 ms.  Rows have nvidia-smi's layout."""
+    timed region of the default run is ~0.3 s), else one `nvidia-smi` query per 100 ms.  Rows have nvidia-smi's layout."""
     Q = ("clocks.sm,clocks.max.sm,clocks_event_reasons.hw_slowdown,clocks_event_reasons.hw_thermal_slowdown,"
          "clocks_event_reasons.sw_thermal_slowdown,clocks_event_reasons.sw_power_cap")
 
@@ -234,7 +259,7 @@ def main():
     os.dup2(2, 1)            # e.g. "NCCL version ..." banners must not precede the JSON line
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=4000)
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=sorted(WORKLOADS))
@@ -242,7 +267,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra-configs", action="store_true", help="measure only --workload (skip the `configs` dict)")
     ap.add_argument("--streams", type=int, default=0, help="execution contexts of the engine (0 = library default 2)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last device-timed step of --workload to DIR/*.npy (--impl b200 only)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path only; it cannot be combined with --impl reference")
     wl = dict(WORKLOADS[args.workload])
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -314,8 +343,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.SUM)
         return float(t[0])
 
-    def measure(name, K, min_s, full):
-        """One workload on this rank's GPU: device-timed and end-to-end numbers as medians over blocks of K steps."""
+    def measure(name, full):
+        """One workload on this rank's GPU: device-timed and end-to-end numbers, each over K timed steps after W warm-up steps."""
         w = dict(WORKLOADS[name])
         prec = precs[w["precision"]]
         B, H, Wd = w["batch"], w["h"], w["w"]
@@ -358,77 +387,71 @@ def main():
 
         def device_step(slot):
             if gather:
-                eng.detect_device_allgather(B, SCORE_THR, NMS_THR, dev[slot].data_ptr())
-            else:
-                eng.detect_device(B, SCORE_THR, NMS_THR, dev[slot].data_ptr())
+                return eng.detect_device_allgather(B, SCORE_THR, NMS_THR, dev[slot].data_ptr())
+            return eng.detect_device(B, SCORE_THR, NMS_THR, dev[slot].data_ptr())
 
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         pos = [0]
+        last = [None]                       # device (dets, counts) of the last device step
 
-        def dev_block():
+        def dev_block(n):
             barrier()
             ev0.record(stream)
-            for _ in range(K):
-                device_step(pos[0] % ring)
+            for _ in range(n):
+                last[0] = device_step(pos[0] % ring)
                 pos[0] += 1
             eng.fence()                     # stream (context 0) now follows the work queued on every context
             ev1.record(stream)
             barrier()
             return ev0.elapsed_time(ev1)
 
-        def e2e_block():
+        def e2e_block(n):
             barrier()
             t0 = time.perf_counter()
-            pipelined(K, pos[0])
-            pos[0] += K
+            pipelined(n, pos[0])
+            pos[0] += n
             barrier()
             return (time.perf_counter() - t0) * 1e3
 
         lat = [None]
 
-        def blk_block():
+        def blk_block(n):
             barrier()
             t0 = time.perf_counter()
-            for _ in range(K):
+            for _ in range(n):
                 lat[0].detect_batch([pin_np[pos[0] % ring, j] for j in range(B)], SCORE_THR, NMS_THR)
                 pos[0] += 1
             barrier()
             return (time.perf_counter() - t0) * 1e3
 
-        def run_blocks(block, warm):
-            """warm-up, then blocks of K steps until >= min_s of timed work on every rank; median block time (max over ranks)."""
-            for _ in range(warm):
-                block()
-            first = agree_max(block())
-            nblk = int(min(400, max(3, -(-min_s * 1e3 // max(first, 1e-3)))))
-            nblk = int(agree_max(nblk))
-            times = [first] + [block() for _ in range(nblk - 1)]
-            times = [agree_max(t) for t in times] if world > 1 else times
-            return float(np.median(times)), len(times), float(np.sum(times)) * 1e-3
+        def timed(block):
+            """W untimed warm-up steps, then exactly K timed steps: their time in ms (max over ranks)."""
+            block(W)
+            return agree_max(block(K))
 
         mean_faces = float(faces_per_slot.mean())          # per step on this rank (the ring is walked round and round)
         faces_step = agree_sum(mean_faces)                 # whole job
-        for i in range(W):
-            device_step(i % ring)
-        barrier()
         out = dict(workload=name, precision=w["precision"], batch_per_gpu=B, input=f"{Wd}x{H}", launches_per_step=eng.launches_per_batch(B))
         clock = None
         if full:
             clock = ClockSampler(local)
             clock.start()
-        d_ms, d_n, d_s = run_blocks(dev_block, 1)
-        out.update(ms_per_step=d_ms / K, value=faces_step * K / (d_ms * 1e-3), images_per_s=K * B * world / (d_ms * 1e-3), timed_blocks=d_n, timed_region_s=d_s)
-        e_ms, e_n, e_s = run_blocks(e2e_block, 1)
+        d_ms = timed(dev_block)
+        out.update(ms_per_step=d_ms / K, value=faces_step * K / (d_ms * 1e-3), images_per_s=K * B * world / (d_ms * 1e-3), timed_region_s=d_ms * 1e-3)
+        if full and args.dump_outputs and rank == 0:
+            eng.synchronize()
+            dump_device_outputs(args.dump_outputs, *last[0], rows, eng.max_faces, f"cuda:{local}")
+        e_ms = timed(e2e_block)
         out["e2e"] = dict(value=faces_step * K / (e_ms * 1e-3), unit="faces/s", h2d_bytes_per_step=img_bytes,
                           d2h_bytes_per_step=(world if gather else 1) * (B * 4 + B * eng.max_faces * 64) + (4 if gather else 0),
-                          images_per_s=K * B * world / (e_ms * 1e-3), ms_per_step=e_ms / K, timed_blocks=e_n, timed_region_s=e_s,
-                          timing=f"host wall clock, median over blocks of K rf_submit_batch{'_allgather' if gather else ''}/rf_collect steps, {depth} batches in flight"
+                          images_per_s=K * B * world / (e_ms * 1e-3), ms_per_step=e_ms / K, timed_region_s=e_ms * 1e-3,
+                          timing=f"host wall clock over {K} rf_submit_batch{'_allgather' if gather else ''}/rf_collect steps, {depth} batches in flight"
                                  + ("; every step's results are the records of ALL ranks, host-visible" if gather else ""))
         if full and not gather:
             # latency mode is its own handle configuration: streams = 1 selects the chain plan (DESIGN.md section 3)
             lat[0] = Engine(os.path.join(GOLD, "weights", w["model"] + ".caffemodel"), H, Wd, precision=prec, max_batch=B, max_faces=128, device=local,
                             streams=1, int8_table=os.path.join(GOLD, "weights", w["model"] + ".table.int8") if prec == RF_PREC_INT8 else None)
-            b_ms, b_n, b_s = run_blocks(blk_block, 1)
+            b_ms = timed(blk_block)
             out["e2e"]["blocking"] = dict(value=faces_step * K / (b_ms * 1e-3), ms_per_step=b_ms / K, images_per_s=K * B * world / (b_ms * 1e-3),
                                           launches_per_step=lat[0].launches_per_batch(B),
                                           note="one blocking rf_detect_batch per step on a streams=1 handle (latency mode: chain plan)")
@@ -443,14 +466,14 @@ def main():
         eng.close()
         return out
 
-    main_res = measure(args.workload, K, MIN_TIMED_S, True)
+    main_res = measure(args.workload, True)
     extras = {}
     if not args.no_extra_configs:
         for name in (EXTRA_NGPU if world > 1 else EXTRA_1GPU):
             if name == args.workload:
                 continue
             try:
-                r = measure(name, K, 0.15, False)
+                r = measure(name, False)
                 extras[name] = {k: v for k, v in r.items() if not k.startswith("_")}
             except Exception as e:                      # a secondary configuration must not take the headline line down
                 extras[name] = dict(error=str(e)[:300])
@@ -484,7 +507,7 @@ def main():
                     dtype={RF_PREC_FP16: "f16", RF_PREC_FP32: "f32", RF_PREC_INT8: "s8"}[prec], data="synthetic",
                     config=dict(config, execution_contexts=args.streams or 8,
                                 l2_policy=f"input ring of {ring} batches = {ring * img_bytes / 2**20:.0f} MiB > 2x L2; activations reused in place",
-                                timing=f"median over {main_res['timed_blocks']} blocks of {K} steps ({main_res['timed_region_s']:.2f} s timed)",
+                                timing=f"{K} timed steps after {W} warm-up steps ({main_res['timed_region_s']:.3f} s timed)",
                                 exchange=("detection records of every step stored into every rank's gather window by the NMS kernel (NVLink peer "
                                           "stores, comm.cu); included in value and e2e") if world > 1 else "none (1 GPU)"),
                     images_per_s=main_res["images_per_s"], clocks=main_res.get("clocks"),

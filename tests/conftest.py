@@ -9,12 +9,10 @@ if ROOT not in sys.path:
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 WEIGHTS = os.path.join(GOLDEN, "weights")
-REFERENCE = "/root/reference"
 
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a B200 (run by the driver with -m gpu)")
-    config.addinivalue_line("markers", "needs_reference: needs /root/reference (this container only)")
 
 
 @pytest.fixture(scope="session")
@@ -34,7 +32,3 @@ def golden_image():
 
 def caffemodel(name: str) -> str:
     return os.path.join(WEIGHTS, name + ".caffemodel")
-
-
-def has_reference() -> bool:
-    return os.path.exists(os.path.join(REFERENCE, "retinaface", "RetinaFace.cpp"))

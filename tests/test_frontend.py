@@ -8,7 +8,7 @@ import shutil
 import numpy as np
 import pytest
 
-from conftest import REFERENCE, caffemodel, has_reference
+from conftest import WEIGHTS, caffemodel
 from oracle import topology
 
 
@@ -28,13 +28,12 @@ def test_generated_prototxt_parses_and_folds_like_the_builtin_graph(gen_prototxt
         assert np.array_equal(w, w0) and np.array_equal(b, b0), layer
 
 
-@pytest.mark.skipif(not has_reference(), reason="/root/reference absent")
 @pytest.mark.parametrize("name,hw", [("mnet25", (416, 288)), ("mnet-deconv-0517", (320, 320))])
 def test_reference_prototxts_are_parsed_from_text(name, hw, built_lib):
     """Both shipped prototxt files (different spellings of the reshape / crop layers, `shape: { ... }` with a colon) parse, pass the
     graph check, give the input size the reference's parseNet reads from line 7, and fold to the same weights as the built-in graph."""
     from retinaface_b200.capi import model_inspect, model_load
-    proto = os.path.join(REFERENCE, "model", name + ".prototxt")
+    proto = os.path.join(WEIGHTS, name + ".prototxt")
     cs, idims, (w, b) = model_load(caffemodel(name), proto, None, "rf_c2_aggr")
     assert idims == (1, 3) + hw
     w0, b0 = model_inspect(caffemodel(name), "rf_c2_aggr")

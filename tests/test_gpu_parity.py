@@ -12,7 +12,7 @@ from conftest import GOLDEN, caffemodel
 from oracle import topology
 from oracle.inputs import letterbox_bgr_u8, s_noise_batch, s_real_batch
 from oracle.mnet_numpy import MnetOracle, preprocess_bgr_u8
-from oracle.postproc import PostprocOracle, ReferencePostproc, synth_heads
+from oracle.postproc import PostprocOracle, synth_heads
 
 pytestmark = pytest.mark.gpu
 
@@ -69,24 +69,25 @@ def test_postprocess_kernels_vs_oracle(post_oracle, hw):
 
 
 def test_postprocess_matches_reference_compiled_code():
-    """Same, against oracle/_ref (the reference's own RetinaFace::postProcess), when it travelled here."""
-    if not ReferencePostproc.available():
-        pytest.skip("oracle/_ref/libref_postproc.so not present")
+    """Same, against what oracle/_ref (the reference's own RetinaFace::postProcess) computed on the same synthetic heads
+    (tests/golden/postproc_reference.npz, written by tests/golden/make_golden.py)."""
+    import hashlib
     from retinaface_b200 import RF_PREC_FP32
     h = w = 448
+    gold = np.load(os.path.join(GOLDEN, "postproc_reference.npz"))
     eng = _engine("mnet25", h, w, RF_PREC_FP32, max_batch=1, max_faces=4096)
-    ref = ReferencePostproc(h, w)
     try:
         for ncand in (5, 300, 2000):
             heads = synth_heads(h, w, ncand, seed=7 + ncand)
+            digest = hashlib.sha256(b"".join(np.ascontiguousarray(x, dtype=np.float32).tobytes() for x in heads)).digest()
+            assert digest == gold[f"gpu_448x448_n{ncand}__heads_sha256"].tobytes(), "synthetic heads differ from those the reference ran on"
             faces, idx, _ = eng.postprocess([x[None] for x in heads], 0.9, 0.4)
-            theirs = ref.postprocess(heads, 0.9)
+            theirs = gold[f"gpu_448x448_n{ncand}"]
             assert faces[0].shape == theirs.shape
             assert np.array_equal(faces[0][:, 0], theirs[:, 0])
             assert np.array_equal(faces[0][:, 5:], theirs[:, 5:])
             assert np.allclose(faces[0][:, 1:5], theirs[:, 1:5], rtol=4e-6, atol=1e-4)
     finally:
-        ref.close()
         eng.close()
 
 

@@ -7,7 +7,7 @@ import tempfile
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, REFERENCE, caffemodel, has_reference
+from conftest import GOLDEN, WEIGHTS, caffemodel
 from oracle import topology
 from oracle.inputs import letterbox_bgr_u8
 from oracle.mnet_numpy import MnetOracle, preprocess_bgr_u8
@@ -45,20 +45,21 @@ def test_generated_prototxt_runs_in_cv2_and_matches_numpy():
         assert np.abs(o - mine[name]).max() < 2e-5, name
 
 
-@pytest.mark.skipif(not has_reference(), reason="/root/reference absent")
 def test_generated_prototxt_equals_reference_prototxt():
+    """cv2.dnn runs the reference's own prototxt (committed byte-identical under tests/golden/weights) and the generated one
+    on the same caffemodel: identical head blobs."""
     import cv2
     rng = np.random.default_rng(4)
     x = preprocess_bgr_u8(rng.integers(0, 256, (96, 64, 3), dtype=np.uint8))
     for model in ("mnet-deconv-0517", "mnet25"):
-        txt = open(f"{REFERENCE}/model/{model}.prototxt").read()
+        txt = open(os.path.join(WEIGHTS, f"{model}.prototxt")).read()
         txt, n = re.subn(r"shape: \{ dim: 1 dim: 3 dim: \d+ dim: \d+ \}", "shape: { dim: 1 dim: 3 dim: 96 dim: 64 }", txt)
         assert n == 1
         with tempfile.TemporaryDirectory() as d:
             pr, pg = os.path.join(d, "r.prototxt"), os.path.join(d, "g.prototxt")
             open(pr, "w").write(txt)
             open(pg, "w").write(topology.to_prototxt(96, 64))
-            a = cv2.dnn.readNetFromCaffe(pr, f"{REFERENCE}/model/{model}.caffemodel")
+            a = cv2.dnn.readNetFromCaffe(pr, caffemodel(model))
             b = cv2.dnn.readNetFromCaffe(pg, caffemodel(model))
             a.setInput(x)
             b.setInput(x)
@@ -66,12 +67,19 @@ def test_generated_prototxt_equals_reference_prototxt():
                 assert np.array_equal(u, v)
 
 
-@pytest.mark.skipif(not has_reference(), reason="/root/reference absent")
 def test_committed_fixtures_are_the_reference_files():
-    import filecmp
-    for f in ("mnet25.caffemodel", "mnet-deconv-0517.caffemodel", "mnet-deconv-0517.table.int8"):
-        assert filecmp.cmp(f"{REFERENCE}/model/{f}", os.path.join(GOLDEN, "weights", f), shallow=False)
-    assert filecmp.cmp(f"{REFERENCE}/data/img.jpg", os.path.join(GOLDEN, "data", "img.jpg"), shallow=False)
+    """Every committed copy of a reference data file has the SHA-256 that file has in the reference
+    (tests/golden/reference_sha256.json, written by tests/golden/make_golden.py)."""
+    import hashlib
+    import json
+    digests = json.load(open(os.path.join(GOLDEN, "reference_sha256.json")))
+    files = {"data/img.jpg": os.path.join(GOLDEN, "data", "img.jpg")}
+    for f in ("mnet25.caffemodel", "mnet-deconv-0517.caffemodel", "mnet25.prototxt", "mnet-deconv-0517.prototxt",
+              "mnet-deconv-0517.table.int8"):
+        files[f"model/{f}"] = os.path.join(WEIGHTS, f)
+    assert sorted(digests) == sorted(files)
+    for name, path in files.items():
+        assert hashlib.sha256(open(path, "rb").read()).hexdigest() == digests[name], name
 
 
 def test_int8_oracle_within_calibration_tolerance_of_fp32(golden_image):

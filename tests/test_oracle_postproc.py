@@ -1,15 +1,29 @@
 """CPU: pins the plain-C post-process restatement (oracle/postproc.c) against the reference's own
-compiled code (oracle/_ref = /root/reference/retinaface/RetinaFace.cpp built unmodified behind a
-fake engine) and against the committed golden detections."""
+compiled code (oracle/_ref: the reference's RetinaFace.cpp built unmodified behind a fake engine), as
+recorded on the same seeded inputs in tests/golden/postproc_reference.npz (tests/golden/make_golden.py),
+and against the committed golden detections."""
+import hashlib
 import os
 
 import numpy as np
 import pytest
 
 from conftest import GOLDEN
-from oracle.postproc import STRIDES, PostprocOracle, ReferencePostproc, synth_heads
+from oracle.postproc import STRIDES, PostprocOracle, synth_heads
 
-needs_ref = pytest.mark.skipif(not ReferencePostproc.available(), reason="oracle/_ref not built (no /root/reference)")
+REF = np.load(os.path.join(GOLDEN, "postproc_reference.npz"))
+
+
+def _sha256(arrays) -> bytes:
+    return hashlib.sha256(b"".join(np.ascontiguousarray(a, dtype=np.float32).tobytes() for a in arrays)).digest()
+
+
+def assert_reference_output(mine: np.ndarray, key: str) -> None:
+    """`mine` is, byte for byte, the array oracle/_ref computed for `key`: same shape, same first rows, same SHA-256."""
+    shape, rows = tuple(REF[key + "__shape"]), REF[key + "__rows"]
+    assert mine.shape == shape, (key, mine.shape, shape)
+    assert np.array_equal(mine[:len(rows)], rows), (key, mine[:len(rows)], rows)
+    assert _sha256([mine]) == REF[key + "__sha256"].tobytes(), key
 
 
 @pytest.fixture(scope="module")
@@ -25,44 +39,36 @@ def test_base_anchors_values(oracle):
         assert oracle.base_anchors(s).tolist() == exp[s]
 
 
-@needs_ref
 @pytest.mark.parametrize("hw", [(448, 448), (896, 1280), (320, 320)])
 def test_anchors_match_reference(oracle, hw):
-    ref = ReferencePostproc(*hw)
-    try:
-        for s in STRIDES:
-            base = oracle.base_anchors(s)
-            assert np.array_equal(base, ref.base_anchors(s))
-            plane = ref.anchor_plane(s)  # anchors_plane: index k*H*W + ih*W + iw
-            h, w = hw[0] // s, hw[1] // s
-            ys, xs = np.mgrid[0:h, 0:w]
-            for k in range(2):
-                mine = np.stack([base[k, 0] + xs * s, base[k, 1] + ys * s, base[k, 2] + xs * s, base[k, 3] + ys * s], -1)
-                assert np.array_equal(mine.reshape(-1, 4).astype(np.float32), plane[k * h * w:(k + 1) * h * w])
-    finally:
-        ref.close()
+    for s in STRIDES:
+        base = oracle.base_anchors(s)
+        assert np.array_equal(base, REF[f"base_{hw[0]}x{hw[1]}_s{s}"])
+        # anchors_plane: index k*H*W + ih*W + iw
+        h, w = hw[0] // s, hw[1] // s
+        ys, xs = np.mgrid[0:h, 0:w]
+        mine = [np.stack([base[k, 0] + xs * s, base[k, 1] + ys * s, base[k, 2] + xs * s, base[k, 3] + ys * s], -1).reshape(-1, 4)
+                for k in range(2)]
+        assert_reference_output(np.concatenate(mine).astype(np.float32), f"plane_{hw[0]}x{hw[1]}_s{s}")
 
 
-@needs_ref
 @pytest.mark.parametrize("hw", [(448, 448), (896, 1280)])
 @pytest.mark.parametrize("ncand", [0, 1, 7, 64, 1024, 4000])
 def test_postprocess_bit_exact_vs_reference(oracle, hw, ncand):
+    key = f"{hw[0]}x{hw[1]}_n{ncand}"
     heads = synth_heads(hw[0], hw[1], ncand, seed=ncand + 11)
-    ref = ReferencePostproc(*hw)
-    try:
-        for thr in (0.9, 0.5):
-            mine = oracle.postprocess(heads, hw[0], hw[1], thr, 0.4)   # reference postProcess hard-codes NMS 0.4
-            theirs = ref.postprocess(heads, thr)
-            assert np.array_equal(mine["faces"], theirs)
-            if thr == 0.9:
-                assert len(mine["cand"]) == ncand
-        # RetinaFace::nms with other thresholds, on the same candidates
-        cands = oracle.postprocess(heads, hw[0], hw[1], 0.9, 0.4)["cand"]
-        for nt in (0.0, 0.3, 0.7, 1.0):
-            a, _ = oracle.nms(cands, nt)
-            assert np.array_equal(a, ref.nms(cands, nt))
-    finally:
-        ref.close()
+    assert _sha256(heads) == REF[f"pp_{key}__heads_sha256"].tobytes(), "synthetic heads differ from those the reference ran on"
+    for thr in (0.9, 0.5):
+        mine = oracle.postprocess(heads, hw[0], hw[1], thr, 0.4)   # reference postProcess hard-codes NMS 0.4
+        assert_reference_output(mine["faces"], f"pp_{key}_thr{thr}")
+        if thr == 0.9:
+            assert len(mine["cand"]) == ncand
+    # RetinaFace::nms with other thresholds, on the same candidates
+    cands = oracle.postprocess(heads, hw[0], hw[1], 0.9, 0.4)["cand"]
+    assert _sha256([cands]) == REF[f"nms_{key}__cands_sha256"].tobytes()
+    for nt in (0.0, 0.3, 0.7, 1.0):
+        a, _ = oracle.nms(cands, nt)
+        assert_reference_output(a, f"nms_{key}_nt{nt}")
 
 
 def test_edge_cases(oracle):
