@@ -154,6 +154,7 @@ int rf_collect_batch(rf_handle h, int ticket, rf_face *out_faces, int *out_count
  * all-gathers (SURVEY.md 8e). */
 int rf_detect_batch_device(rf_handle h, const uint8_t *dev_bgr, int n, float score_threshold,
                            float nms_threshold, const rf_det **dev_dets, const int32_t **dev_counts);
+/* (aligned crops of these results: rf_align_batch_device, below) */
 
 /* f1 ingest, compressed: the reference decodes its test images on the host (cv::imread, main.cpp:18-26) and then copies
  * pixels; here the JPEG bitstreams are decoded ON the GPU (nvJPEG, opened at run time; hardware JPEG engines when the device
@@ -226,6 +227,38 @@ typedef struct rf_view {
 int rf_detect_views(rf_handle h, const uint8_t *bgr, int width, int height, int row_stride, const rf_view *views, int nviews,
                     float score_threshold, float nms_threshold, rf_face *out_faces, int *out_count, int32_t *out_view_of,
                     float *out_view_scales);
+
+/* Landmark-aligned face crops: insightface's norm_crop -- a similarity transform fitted (least squares, no reflection, FP64)
+ * from a face's five landmarks to a template, then cv2.warpAffine(img, M, (crop_w, crop_h), INTER_LINEAR, BORDER_CONSTANT, 0)
+ * -- on the GPU, byte for byte what OpenCV computes with the same M.  The crop is what a recognizer (ArcFace and its relatives)
+ * takes.  One kernel launch per call aligns the first min(count, max_crops) faces of every image, in score order, straight
+ * from the full-resolution source images the detector read; it is not part of the forward graph. */
+#define RF_CROP_U8_BGR  0   /* [crop_h][crop_w][3] u8 BGR: norm_crop's output */
+#define RF_CROP_F16_RGB 1   /* [3][crop_h][crop_w] FP16 of (v - mean) * scale, RGB planes: a recognizer's input tensor */
+typedef struct rf_align_spec {
+    int crop_w, crop_h;         /* 1..1024; with the default template both must be multiples of 112 */
+    float dst_x[5], dst_y[5];   /* landmark template in crop pixels; all zero -> the ArcFace 112 template scaled by crop / 112
+                                   (insightface estimate_norm) */
+    int max_crops;              /* per image, 1..max_faces: crops of the top-scoring faces */
+    int layout;                 /* RF_CROP_* */
+    float mean, scale;          /* RF_CROP_F16_RGB only (insightface: 127.5, 1/127.5) */
+} rf_align_spec;
+
+/* rf_detect_batch + aligned crops of the first min(out_counts[i], max_crops) faces of each image, sampled from the caller's
+ * ORIGINAL image (any size <= max_image; at most raw_slots -- max_batch, capped at 2 GiB of image buffers -- of them not
+ * network-sized, RF_ERR_CAPACITY otherwise).  Faces / counts / anchor indices exactly as rf_detect_batch (network-input
+ * pixels); out_scales (optional) [n]: the map-back factor to image pixels; out_crops (host) [n][max_crops][crop] in the spec's
+ * layout; out_affine (optional) [n][max_crops][6] doubles, the image -> crop matrix of each crop.  Slots past the count are not
+ * written.  Blocking. */
+int rf_detect_align_batch(rf_handle h, const uint8_t *const *bgr_images, const int *widths, const int *heights,
+                          const int *row_strides, int n, float score_threshold, float nms_threshold, const rf_align_spec *spec,
+                          rf_face *out_faces, int *out_counts, int32_t *out_anchor_index, float *out_scales,
+                          void *out_crops, double *out_affine);
+/* Device-resident: after rf_detect_batch_device(h, dev_bgr, n, ...) align from the same network-sized device images and the
+ * records it returned (dev_dets [n][max_faces], dev_counts [n]).  Enqueued on rf_last_stream(); dev_crops / dev_affine
+ * (optional) are caller-owned device memory laid out as above; slots past the count are not written. */
+int rf_align_batch_device(rf_handle h, const uint8_t *dev_bgr, int n, const rf_det *dev_dets, const int32_t *dev_counts,
+                          const rf_align_spec *spec, void *dev_crops, double *dev_affine);
 
 /* Preprocess parity: replaces imageROIResize8U3C + the OpenCV branch (RetinaFace.cpp:593-647):
  * letter-boxes one host image into a host net_h*net_w*3 u8 BGR buffer using the GPU kernel. */

@@ -24,6 +24,7 @@ SOURCES = [
     ("jpeg.cu", []),
     ("postproc.cu", ["-fmad=false"]),
     ("preprocess.cu", ["-fmad=false"]),
+    ("align.cu", ["-fmad=false"]),
     ("calibrate.cu", []),
     ("model.cpp", []),
     ("frontend.cpp", []),

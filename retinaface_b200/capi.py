@@ -26,12 +26,40 @@ EXPORTS = [
     "rf_submit_batch_allgather", "rf_collect_batch_allgather", "rf_detect_batch_allgather",
     "rf_model_load", "rf_network_config", "rf_cache_status",
     "rf_detect_jpeg_batch", "rf_decode_jpeg", "rf_jpeg_backend",
+    "rf_detect_align_batch", "rf_align_batch_device",
 ]
 COMM_BLOB_BYTES = 128
 
 
 class _View(C.Structure):       # rf_view
     _fields_ = [("shrink", C.c_float), ("flip", C.c_int32)]
+
+
+RF_CROP_U8_BGR, RF_CROP_F16_RGB = 0, 1
+# insightface's arcface_dst: the five-landmark template of a 112 x 112 recognizer crop (crop pixels, float32)
+ARCFACE_112 = np.array([[38.2946, 51.6963], [73.5318, 51.5014], [56.0252, 71.7366], [41.5493, 92.3655], [70.7299, 92.2041]],
+                       dtype=np.float32)
+
+
+class _AlignSpec(C.Structure):  # rf_align_spec
+    _fields_ = [("crop_w", C.c_int), ("crop_h", C.c_int), ("dst_x", C.c_float * 5), ("dst_y", C.c_float * 5),
+                ("max_crops", C.c_int), ("layout", C.c_int), ("mean", C.c_float), ("scale", C.c_float)]
+
+
+def align_spec(crop: Tuple[int, int] = (112, 112), template=None, max_crops: int = 16, layout: int = RF_CROP_U8_BGR,
+               mean: float = 127.5, scale: float = float(np.float32(1 / 127.5))) -> _AlignSpec:
+    """rf_align_spec: crop = (width, height); template = (5, 2) landmark positions in crop pixels, None -> the ArcFace template
+    scaled by crop / 112 (sides must then be multiples of 112); mean / scale apply to RF_CROP_F16_RGB."""
+    t = np.zeros((5, 2), dtype=np.float32) if template is None else np.asarray(template, dtype=np.float32).reshape(5, 2)
+    return _AlignSpec(int(crop[0]), int(crop[1]), (C.c_float * 5)(*t[:, 0]), (C.c_float * 5)(*t[:, 1]), int(max_crops), int(layout),
+                      float(mean), float(scale))
+
+
+def crop_shape(spec: _AlignSpec) -> Tuple[Tuple[int, ...], type]:
+    """(shape, dtype) of one crop in the spec's layout."""
+    if spec.layout == RF_CROP_F16_RGB:
+        return (3, spec.crop_h, spec.crop_w), np.float16
+    return (spec.crop_h, spec.crop_w, 3), np.uint8
 
 
 class RfError(RuntimeError):
@@ -115,6 +143,11 @@ def load_library() -> C.CDLL:
                                          C.c_void_p, C.c_void_p]
     lib.rf_decode_jpeg.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]
     lib.rf_jpeg_backend.restype = C.c_char_p
+    lib.rf_detect_align_batch.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_int,
+                                          C.c_float, C.c_float, C.POINTER(_AlignSpec), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_void_p, C.c_void_p]
+    lib.rf_align_batch_device.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(_AlignSpec), C.c_void_p,
+                                          C.c_void_p]
     lib.rf_jpeg_backend.argtypes = [C.c_void_p]
     _lib = lib
     return lib
@@ -298,6 +331,51 @@ class Engine:
         if want_index:
             return out, [idx[i, :counts[i]].copy() for i in range(n)]
         return out
+
+    def detect_align(self, images: Sequence[np.ndarray], thr: float, nms_thr: float, crop: Tuple[int, int] = (112, 112), template=None,
+                     max_crops: int = 16, layout: int = RF_CROP_U8_BGR, want_index: bool = False, spec: Optional[_AlignSpec] = None):
+        """rf_detect_align_batch: detect_batch + the aligned crops of the top min(count, max_crops) faces of each image, sampled
+        from the original image.  images: u8 BGR HWC arrays (rows may be padded: any view with pixel stride 3).  Returns
+        (per image (faces (k, 15) in network-input pixels, crops (m, ...) in the layout of crop_shape, affine (m, 2, 3) image ->
+        crop), map-back scales (n,)) [+ anchor-index arrays]."""
+        spec = spec if spec is not None else align_spec(crop, template, max_crops, layout)
+        n = len(images)
+        keep = []
+        for im in images:
+            if im.ndim != 3 or im.shape[2] != 3:
+                raise ValueError(f"u8 BGR HWC images expected, got shape {im.shape}")
+            if im.dtype != np.uint8 or im.strides[1:] != (3, 1) or im.strides[0] < 3 * im.shape[1]:
+                im = np.ascontiguousarray(im, dtype=np.uint8)
+            keep.append(im)
+        ptrs = (C.c_void_p * n)(*[im.ctypes.data for im in keep])
+        ws = (C.c_int * n)(*[im.shape[1] for im in keep])
+        hs = (C.c_int * n)(*[im.shape[0] for im in keep])
+        rs = (C.c_int * n)(*[im.strides[0] for im in keep])
+        shape, dt = crop_shape(spec)
+        mc = spec.max_crops
+        faces = np.empty((n, self.max_faces, FACE_FLOATS), dtype=np.float32)
+        counts = np.zeros(n, dtype=np.int32)
+        idx = np.empty((n, self.max_faces), dtype=np.int32)
+        scales = np.empty(n, dtype=np.float32)
+        crops = np.empty((n, mc) + shape, dtype=dt)
+        affine = np.empty((n, mc, 2, 3), dtype=np.float64)
+        self._check(self.lib.rf_detect_align_batch(self.h, ptrs, ws, hs, rs, n, thr, nms_thr, C.byref(spec), faces.ctypes.data,
+                                                   counts.ctypes.data, idx.ctypes.data, scales.ctypes.data, crops.ctypes.data,
+                                                   affine.ctypes.data))
+        out = []
+        for i in range(n):
+            m = min(int(counts[i]), mc)
+            out.append((faces[i, :counts[i]].copy(), crops[i, :m].copy(), affine[i, :m].copy()))
+        if want_index:
+            return out, scales, [idx[i, :counts[i]].copy() for i in range(n)]
+        return out, scales
+
+    def align_device(self, n: int, dev_images_ptr: int, dets_ptr: int, counts_ptr: int, out_ptr: int, spec: _AlignSpec,
+                     affine_ptr: Optional[int] = None):
+        """rf_align_batch_device: aligned crops of the records of a detect_device() call on the same network-sized device images,
+        written to caller device memory out_ptr ([n][max_crops][crop], e.g. a torch CUDA tensor's data_ptr()) and, optionally,
+        the image -> crop matrices to affine_ptr ([n][max_crops][6] doubles).  Asynchronous on last_stream_ptr()."""
+        self._check(self.lib.rf_align_batch_device(self.h, dev_images_ptr, n, dets_ptr, counts_ptr, C.byref(spec), out_ptr, affine_ptr))
 
     def detect_jpeg(self, streams: Sequence[bytes], thr: float, nms_thr: float):
         """JPEG bitstreams (bytes) -> decoded on the GPU (nvJPEG), letter-boxed, detected.  Returns (list of (k,15) arrays in

@@ -5,6 +5,7 @@
 // (retinaface/tensorrt/trtnetbase.cpp:199-330, trtretinafacenet.cpp:48-210) and the detect
 // orchestration of RetinaFace::detect / detectBatchImages (retinaface/RetinaFace.cpp:576-940).
 #include "engine_internal.cuh"
+#include "align.cuh"
 #include "calibrate.cuh"
 #include "preprocess.cuh"
 
@@ -176,6 +177,7 @@ void destroy(rf_handle h) {
     for (auto p : h->d_blobs) cudaFree(p);
     h->copy_pool.reset();
     for (auto e : h->raw_ev) if (e) cudaEventDestroy(e);
+    cudaFree(h->d_crops); cudaFree(h->d_affine); cudaFree(h->d_align_src); cudaFreeHost(h->h_align_src);
     cudaFreeHost(h->h_input); cudaFreeHost(h->h_raw); cudaFreeHost(h->h_dets); cudaFreeHost(h->h_counts); cudaFreeHost(h->tile_dbg);
     for (auto &sl : h->slots) {
         cudaFree(sl.d_in); cudaFreeHost(sl.h_in); cudaFreeHost(sl.h_dets); cudaFreeHost(sl.h_counts);
@@ -524,74 +526,205 @@ static uint8_t *upload_raw(rf_handle h, const uint8_t *src, int width, int heigh
     return d_dst;
 }
 
+// Input staging of one call of caller images (rf_detect_batch, rf_detect_align_batch) into d_input on the handle's stream.
+// Network-sized packed images are copied H2D straight from the caller's memory when it is pinned (cudaHostAlloc /
+// cudaHostRegister / the library's own rf_pinned_input), otherwise via the library's pinned mirror; runs of adjacent sources
+// collapse into one copy.  Other sizes are uploaded into per-image raw buffers and letter-boxed by ONE launch for all of them
+// (preprocess.cuh; RF_FLAG_NPP_RESIZE: the reference's NPP super-sampling definition instead of its OpenCV bilinear one).
+// More than raw_slots letter-boxed images reuse the raw buffers chunk by chunk.  srcs / scales (optional, [n]): where each
+// image's original pixels are on the device -- still there after the forward only when no raw buffer was reused, which
+// rf_detect_align_batch checks before it calls this -- and the reference's map-back factor.
+static int stage_inputs(rf_handle h, const char *who, const uint8_t *const *imgs, const int *widths, const int *heights,
+                        const int *row_strides, int n, AlignSrc *srcs, float *scales) {
+    const int Hn = h->cfg.net_h, Wn = h->cfg.net_w;
+    const size_t img_bytes = (size_t)Hn * Wn * 3;
+    const uint8_t *run_src = nullptr;
+    int run_start = -1, run_len = 0;
+    auto flush = [&]() {
+        if (run_start < 0) return;
+        CK(cudaMemcpyAsync(h->d_input + (size_t)run_start * img_bytes, run_src, (size_t)run_len * img_bytes,
+                           cudaMemcpyHostToDevice, h->stream));
+        run_start = -1;
+    };
+    bool staging_dirty = false;
+    const int area = (h->cfg.flags & RF_FLAG_NPP_RESIZE) ? 1 : 0;
+    std::vector<LbItem> lb;
+    auto flush_lb = [&]() {
+        if (lb.empty()) return;
+        CK(launch_letterbox_batch(lb.data(), (int)lb.size(), Wn, Hn, h->stream));
+        lb.clear();
+    };
+    for (int i = 0; i < n; i++) {
+        if (!imgs[i] || widths[i] <= 0 || heights[i] <= 0) { return fail(h, RF_ERR_INVALID_ARG, fmt("%s: image %d is empty", who, i)); }
+        const int rs = row_strides && row_strides[i] ? row_strides[i] : widths[i] * 3;
+        if (widths[i] == Wn && heights[i] == Hn && rs == Wn * 3) {
+            const uint8_t *src = imgs[i];
+            const bool in_mirror = src >= h->h_input && src < h->h_input + (size_t)h->cfg.max_batch * img_bytes;
+            if (!in_mirror) {
+                cudaPointerAttributes at{};
+                bool pinned = cudaPointerGetAttributes(&at, src) == cudaSuccess && at.type == cudaMemoryTypeHost;
+                if (!pinned) {
+                    cudaGetLastError();
+                    if (!staging_dirty) { CK(cudaStreamSynchronize(h->stream)); staging_dirty = true; }
+                    uint8_t *slot = h->h_input + (size_t)i * img_bytes;
+                    memcpy(slot, src, img_bytes);
+                    src = slot;
+                }
+            }
+            if (run_start >= 0 && src == run_src + (size_t)run_len * img_bytes) { run_len++; }
+            else { flush(); run_start = i; run_src = src; run_len = 1; }
+            if (srcs) srcs[i] = AlignSrc{h->d_input + (size_t)i * img_bytes, Wn, Hn, Wn * 3, 1.f};
+            if (scales) scales[i] = 1.f;
+        } else {
+            flush();
+            if (widths[i] > h->cfg.max_image_w || heights[i] > h->cfg.max_image_h)
+                return fail(h, RF_ERR_CAPACITY, fmt("image %d is %dx%d, larger than max_image %dx%d", i, widths[i], heights[i],
+                                                    h->cfg.max_image_w, h->cfg.max_image_h));
+            if ((int)lb.size() == h->raw_slots) flush_lb();
+            const uint8_t *d_src = upload_raw(h, imgs[i], widths[i], heights[i], rs, (int)lb.size());
+            lb.emplace_back();
+            const float sc = letterbox_fill(lb.back(), d_src, widths[i], heights[i], h->d_input + (size_t)i * img_bytes, Wn, Hn, 0, area);
+            if (srcs) srcs[i] = AlignSrc{d_src, widths[i], heights[i], widths[i] * 3, sc};
+            if (scales) scales[i] = sc;
+        }
+    }
+    flush();
+    flush_lb();
+    return RF_OK;
+}
+
 int rf_detect_batch(rf_handle h, const uint8_t *const *imgs, const int *widths, const int *heights, const int *row_strides,
                     int n, float thr, float nms, rf_face *out_faces, int *out_counts, int32_t *out_idx) {
     int rc = check_n(h, n);
     if (rc) return rc;
     if (n == 0) return RF_OK;
     if (!imgs || !widths || !heights) return fail(h, RF_ERR_INVALID_ARG, "rf_detect_batch: NULL image arrays");
-    const int Hn = h->cfg.net_h, Wn = h->cfg.net_w;
-    const size_t img_bytes = (size_t)Hn * Wn * 3;
     try {
         CK(cudaSetDevice(h->device));
         switch_ctx(h, 0);
-        // Network-sized packed images are copied H2D straight from the caller's memory when it is
-        // pinned (cudaHostAlloc / cudaHostRegister / the library's own rf_pinned_input), otherwise via the
-        // library's pinned mirror; runs of adjacent sources collapse into one copy.  Other sizes are
-        // letter-boxed on the GPU one by one (preprocess.cuh).
-        const uint8_t *run_src = nullptr;
-        int run_start = -1, run_len = 0;
-        auto flush = [&]() {
-            if (run_start < 0) return;
-            CK(cudaMemcpyAsync(h->d_input + (size_t)run_start * img_bytes, run_src, (size_t)run_len * img_bytes,
-                               cudaMemcpyHostToDevice, h->stream));
-            run_start = -1;
-        };
-        bool staging_dirty = false;
-        // other sizes: uploaded into per-image raw buffers, then ONE letter-box launch for all of them (RF_FLAG_NPP_RESIZE: the
-        // reference's NPP super-sampling definition instead of its OpenCV bilinear one)
-        const int area = (h->cfg.flags & RF_FLAG_NPP_RESIZE) ? 1 : 0;
-        std::vector<LbItem> lb;
-        auto flush_lb = [&]() {
-            if (lb.empty()) return;
-            CK(launch_letterbox_batch(lb.data(), (int)lb.size(), Wn, Hn, h->stream));
-            lb.clear();
-        };
-        for (int i = 0; i < n; i++) {
-            if (!imgs[i] || widths[i] <= 0 || heights[i] <= 0) { return fail(h, RF_ERR_INVALID_ARG, fmt("rf_detect_batch: image %d is empty", i)); }
-            const int rs = row_strides && row_strides[i] ? row_strides[i] : widths[i] * 3;
-            if (widths[i] == Wn && heights[i] == Hn && rs == Wn * 3) {
-                const uint8_t *src = imgs[i];
-                const bool in_mirror = src >= h->h_input && src < h->h_input + (size_t)h->cfg.max_batch * img_bytes;
-                if (!in_mirror) {
-                    cudaPointerAttributes at{};
-                    bool pinned = cudaPointerGetAttributes(&at, src) == cudaSuccess && at.type == cudaMemoryTypeHost;
-                    if (!pinned) {
-                        cudaGetLastError();
-                        if (!staging_dirty) { CK(cudaStreamSynchronize(h->stream)); staging_dirty = true; }
-                        uint8_t *slot = h->h_input + (size_t)i * img_bytes;
-                        memcpy(slot, src, img_bytes);
-                        src = slot;
-                    }
-                }
-                if (run_start >= 0 && src == run_src + (size_t)run_len * img_bytes) { run_len++; }
-                else { flush(); run_start = i; run_src = src; run_len = 1; }
-            } else {
-                flush();
-                if (widths[i] > h->cfg.max_image_w || heights[i] > h->cfg.max_image_h)
-                    return fail(h, RF_ERR_CAPACITY, fmt("image %d is %dx%d, larger than max_image %dx%d", i, widths[i], heights[i],
-                                                        h->cfg.max_image_w, h->cfg.max_image_h));
-                if ((int)lb.size() == h->raw_slots) flush_lb();
-                const uint8_t *d_src = upload_raw(h, imgs[i], widths[i], heights[i], rs, (int)lb.size());
-                lb.emplace_back();
-                letterbox_fill(lb.back(), d_src, widths[i], heights[i], h->d_input + (size_t)i * img_bytes, Wn, Hn, 0, area);
-            }
-        }
-        flush();
-        flush_lb();
+        if ((rc = stage_inputs(h, "rf_detect_batch", imgs, widths, heights, row_strides, n, nullptr, nullptr))) return rc;
         set_params(h, thr, nms);
         forward_graph(h, n);
         fetch_results(h, n, out_faces, out_counts, out_idx, nullptr);
+    } catch (const CudaFail &f) { return fail_cuda(h, f); }
+    return RF_OK;
+}
+
+// ---- aligned face crops (align.cuh) -------------------------------------------------------------------------------------------
+// insightface's ArcFace template (arcface_dst, float32) of a 112 x 112 crop
+static const float kArcface112[5][2] = {{38.2946f, 51.6963f}, {73.5318f, 51.5014f}, {56.0252f, 71.7366f}, {41.5493f, 92.3655f}, {70.7299f, 92.2041f}};
+
+// Checks a spec and fills the geometry / template / layout part of the kernel arguments.
+static int align_args(rf_handle h, const char *who, const rf_align_spec *spec, AlignArgs &a) {
+    if (!spec) return fail(h, RF_ERR_INVALID_ARG, fmt("%s: NULL rf_align_spec", who));
+    if (spec->crop_w <= 0 || spec->crop_h <= 0 || spec->crop_w > ALIGN_MAX_CROP || spec->crop_h > ALIGN_MAX_CROP)
+        return fail(h, RF_ERR_INVALID_ARG, fmt("%s: crop %dx%d, each side must be in 1..%d", who, spec->crop_w, spec->crop_h, ALIGN_MAX_CROP));
+    if (spec->max_crops < 1 || spec->max_crops > h->cfg.max_faces)
+        return fail(h, RF_ERR_INVALID_ARG, fmt("%s: max_crops %d outside 1..max_faces (%d)", who, spec->max_crops, h->cfg.max_faces));
+    if (spec->layout != RF_CROP_U8_BGR && spec->layout != RF_CROP_F16_RGB)
+        return fail(h, RF_ERR_INVALID_ARG, fmt("%s: unknown crop layout %d", who, spec->layout));
+    a = AlignArgs{};
+    bool zero = true;
+    for (int k = 0; k < 5; k++) zero = zero && spec->dst_x[k] == 0.f && spec->dst_y[k] == 0.f;
+    if (zero) {
+        if (spec->crop_w % 112 || spec->crop_h % 112)
+            return fail(h, RF_ERR_INVALID_ARG, fmt("%s: the default (ArcFace) template needs crop sides that are multiples of 112, got %dx%d; "
+                                                   "pass a template for other sizes", who, spec->crop_w, spec->crop_h));
+        const float fx = (float)(spec->crop_w / 112.0), fy = (float)(spec->crop_h / 112.0);   // estimate_norm: template * size / 112
+        for (int k = 0; k < 5; k++) { a.dst_x[k] = kArcface112[k][0] * fx; a.dst_y[k] = kArcface112[k][1] * fy; }
+    } else {
+        for (int k = 0; k < 5; k++) { a.dst_x[k] = spec->dst_x[k]; a.dst_y[k] = spec->dst_y[k]; }
+    }
+    a.crop_w = spec->crop_w; a.crop_h = spec->crop_h; a.layout = spec->layout;
+    a.max_crops = spec->max_crops; a.max_faces = h->cfg.max_faces;
+    a.mean = spec->mean; a.scale = spec->scale;
+    return RF_OK;
+}
+
+static size_t crop_bytes(const AlignArgs &a) { return (size_t)a.crop_w * a.crop_h * 3 * (a.layout == RF_CROP_F16_RGB ? 2 : 1); }
+
+int rf_detect_align_batch(rf_handle h, const uint8_t *const *imgs, const int *widths, const int *heights, const int *row_strides, int n,
+                          float thr, float nms, const rf_align_spec *spec, rf_face *out_faces, int *out_counts, int32_t *out_idx,
+                          float *out_scales, void *out_crops, double *out_affine) {
+    static const char *who = "rf_detect_align_batch";
+    int rc = check_n(h, n);
+    if (rc) return rc;
+    AlignArgs a;
+    if ((rc = align_args(h, who, spec, a))) return rc;
+    if (n == 0) return RF_OK;
+    if (!imgs || !widths || !heights || !out_crops) return fail(h, RF_ERR_INVALID_ARG, fmt("%s: NULL image arrays or out_crops", who));
+    // the crops are sampled from the raw buffers after the forward: every letter-boxed image of the call needs its own
+    int lettered = 0;
+    for (int i = 0; i < n; i++) {
+        const int rs = row_strides && row_strides[i] ? row_strides[i] : widths[i] * 3;
+        lettered += !(widths[i] == h->cfg.net_w && heights[i] == h->cfg.net_h && rs == h->cfg.net_w * 3);
+    }
+    if (lettered > h->raw_slots)
+        return fail(h, RF_ERR_CAPACITY, fmt("%s: %d images are not network-sized; the handle keeps at most %d original images on the device "
+                                            "(raw_slots: max_batch, capped at 2 GiB of max_image buffers)", who, lettered, h->raw_slots));
+    const size_t cb = crop_bytes(a);
+    try {
+        CK(cudaSetDevice(h->device));
+        switch_ctx(h, 0);
+        const size_t slots = (size_t)h->cfg.max_batch * a.max_crops;
+        if (slots * cb > h->crops_bytes || slots > h->affine_count) {
+            CK(cudaStreamSynchronize(h->stream));
+            CK(cudaFree(h->d_crops)); h->d_crops = nullptr;
+            CK(cudaFree(h->d_affine)); h->d_affine = nullptr;
+            h->crops_bytes = std::max(h->crops_bytes, slots * cb);
+            h->affine_count = std::max(h->affine_count, slots);
+            CK(cudaMalloc(&h->d_crops, h->crops_bytes));
+            CK(cudaMalloc(&h->d_affine, sizeof(double) * 6 * h->affine_count));
+        }
+        if (!h->d_align_src) {
+            CK(cudaMalloc(&h->d_align_src, sizeof(AlignSrc) * h->cfg.max_batch));
+            CK(cudaHostAlloc(&h->h_align_src, sizeof(AlignSrc) * h->cfg.max_batch, cudaHostAllocDefault));
+        }
+        std::vector<float> scales(n);
+        if ((rc = stage_inputs(h, who, imgs, widths, heights, row_strides, n, h->h_align_src, scales.data()))) return rc;
+        CK(cudaMemcpyAsync(h->d_align_src, h->h_align_src, sizeof(AlignSrc) * n, cudaMemcpyHostToDevice, h->stream));
+        set_params(h, thr, nms);
+        forward_graph(h, n);
+        a.table = h->d_align_src;
+        a.dets = h->pb.out_dets;
+        a.counts = h->pb.out_counts;
+        a.crops = h->d_crops;
+        a.affine = h->d_affine;
+        CK(launch_align(a, n, h->stream));
+        fetch_results(h, n, out_faces, out_counts, out_idx, nullptr);
+        // only the crops that exist cross PCIe
+        for (int i = 0; i < n; i++) {
+            const size_t k = (size_t)std::min(h->h_counts[i], a.max_crops), c0 = (size_t)i * a.max_crops;
+            if (!k) continue;
+            CK(cudaMemcpyAsync(static_cast<uint8_t *>(out_crops) + c0 * cb, h->d_crops + c0 * cb, k * cb, cudaMemcpyDeviceToHost, h->stream));
+            if (out_affine) CK(cudaMemcpyAsync(out_affine + c0 * 6, h->d_affine + c0 * 6, k * 6 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+        }
+        CK(cudaStreamSynchronize(h->stream));
+        if (out_scales) for (int i = 0; i < n; i++) out_scales[i] = scales[i];
+    } catch (const CudaFail &f) { return fail_cuda(h, f); }
+    return RF_OK;
+}
+
+int rf_align_batch_device(rf_handle h, const uint8_t *dev_bgr, int n, const rf_det *dev_dets, const int32_t *dev_counts,
+                          const rf_align_spec *spec, void *dev_crops, double *dev_affine) {
+    static const char *who = "rf_align_batch_device";
+    int rc = check_n(h, n);
+    if (rc) return rc;
+    AlignArgs a;
+    if ((rc = align_args(h, who, spec, a))) return rc;
+    if (n == 0) return RF_OK;
+    if (!dev_bgr || !dev_dets || !dev_counts || !dev_crops) return fail(h, RF_ERR_INVALID_ARG, fmt("%s: NULL device pointer", who));
+    const int Hn = h->cfg.net_h, Wn = h->cfg.net_w;
+    try {
+        CK(cudaSetDevice(h->device));
+        a.table = nullptr;
+        a.uniform = AlignSrc{dev_bgr, Wn, Hn, Wn * 3, 1.f};
+        a.uniform_stride = (size_t)Hn * Wn * 3;
+        a.dets = dev_dets;
+        a.counts = dev_counts;
+        a.crops = dev_crops;
+        a.affine = dev_affine;
+        CK(launch_align(a, n, h->last_stream ? h->last_stream : h->stream));   // the stream rf_last_stream() reports
     } catch (const CudaFail &f) { return fail_cuda(h, f); }
     return RF_OK;
 }

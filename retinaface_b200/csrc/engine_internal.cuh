@@ -15,6 +15,7 @@
 #include <type_traits>
 #include <vector>
 
+#include "align.cuh"
 #include "common.cuh"
 #include "host_copy.h"
 #include "model.h"
@@ -143,6 +144,11 @@ struct rf_handle_s {
     rf_det *h_dets = nullptr;         // pinned [max_batch][max_faces]
     int *h_counts = nullptr;          // pinned [2*max_batch]: kept, candidates
     std::map<int, cudaGraphExec_t> graphs;
+    // aligned crops of rf_detect_align_batch (context 0; lazily allocated, regrown when a spec needs more)
+    uint8_t *d_crops = nullptr;       // [max_batch][max_crops][crop]
+    double *d_affine = nullptr;       // [max_batch][max_crops][6]
+    size_t crops_bytes = 0, affine_count = 0;
+    AlignSrc *d_align_src = nullptr, *h_align_src = nullptr;   // [max_batch] source table of the align kernel (device, pinned)
     // pipelined end-to-end path (rf_submit_batch / rf_collect_batch)
     struct Slot {
         uint8_t *d_in = nullptr, *h_in = nullptr;     // device input, pinned staging for pageable sources

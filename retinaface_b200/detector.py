@@ -10,7 +10,7 @@ from __future__ import annotations
 
 import os
 from dataclasses import dataclass
-from typing import List, Sequence
+from typing import List, Sequence, Tuple
 
 import numpy as np
 
@@ -63,6 +63,25 @@ class RetinaFace:
         views = [(float(s), f) for s in scales for f in ((False, True) if flip else (False,))]
         faces, _, _ = self.engine.detect_views(img, views, threshold, self.nms_threshold)
         return [FaceDetectInfo.from_row(r) for r in faces]
+
+    def detectAndAlign(self, imgs: Sequence[np.ndarray], threshold: float = 0.5, crop_size: int = 112,
+                       max_crops: int = 16) -> List[List[Tuple[FaceDetectInfo, np.ndarray]]]:
+        """Detection + the step a recognition pipeline takes next (insightface's norm_crop): per image, up to ``max_crops``
+        faces in score order as (FaceDetectInfo in ORIGINAL IMAGE pixels, aligned crop_size x crop_size u8 BGR crop).  The
+        crops are warped on the GPU (rf_detect_align_batch) from the original images, byte-identical to cv2.warpAffine with
+        the ArcFace-template similarity of the face's landmarks; ``crop_size`` must be a multiple of 112."""
+        out: List[List[Tuple[FaceDetectInfo, np.ndarray]]] = []
+        imgs = list(imgs)
+        mb = self.engine.max_batch
+        for start in range(0, len(imgs), mb):
+            per, scales = self.engine.detect_align(imgs[start:start + mb], threshold, self.nms_threshold, crop=(crop_size, crop_size),
+                                                   max_crops=max_crops)
+            for (faces, crops, _), s in zip(per, scales):
+                s = np.float32(s)
+                rows = faces[:len(crops)].copy()
+                rows[:, 1:] *= s        # network-input -> image pixels (RetinaFace.cpp:732-738), in float32 like the library
+                out.append([(FaceDetectInfo.from_row(r), c) for r, c in zip(rows, crops)])
+        return out
 
     @staticmethod
     def draw(img: np.ndarray, faces: Sequence[FaceDetectInfo]) -> np.ndarray:

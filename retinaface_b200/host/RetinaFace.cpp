@@ -1,7 +1,9 @@
 // RetinaFace.cpp -- see RetinaFace.h.  Everything that computes lives behind the C ABI.
 #include "RetinaFace.h"
 
+#include <algorithm>
 #include <cmath>
+#include <cstring>
 
 #include <stdexcept>
 
@@ -92,6 +94,40 @@ void RetinaFace::detectBatchImages(vector<cv::Mat> imgs, float threshold) {
         for (int i = 0; i < n; i++) {
             const FaceDetectInfo *f = reinterpret_cast<const FaceDetectInfo *>(out_faces_.data() + (size_t)i * opt_.max_faces);
             last_[start + i].assign(f, f + out_counts_[i]);
+        }
+    }
+}
+
+void RetinaFace::detectAndAlign(vector<cv::Mat> imgs, float threshold) {
+    last_.assign(imgs.size(), vector<FaceDetectInfo>());
+    scales_.assign(imgs.size(), 1.f);
+    crops_.assign(imgs.size(), vector<Mat>());
+    rf_align_spec spec{};             // zero template: the ArcFace one, scaled by crop_size / 112
+    spec.crop_w = spec.crop_h = opt_.crop_size;
+    spec.max_crops = opt_.max_crops;
+    spec.layout = RF_CROP_U8_BGR;
+    const size_t mb = (size_t)opt_.max_batch, crop_bytes = (size_t)opt_.crop_size * opt_.crop_size * 3;
+    vector<unsigned char> crops(mb * (size_t)opt_.max_crops * crop_bytes);
+    for (size_t start = 0; start < imgs.size(); start += mb) {
+        const int n = (int)std::min(mb, imgs.size() - start);
+        vector<const uint8_t *> ptrs(n);
+        vector<int> ws(n), hs(n), strides(n);
+        for (int i = 0; i < n; i++) {
+            const cv::Mat &m = imgs[start + i];
+            if (m.empty()) throw std::runtime_error("detectAndAlign: empty image");
+            ptrs[i] = m.data; ws[i] = m.cols; hs[i] = m.rows; strides[i] = (int)m.step;
+        }
+        int rc = rf_detect_align_batch(h_, ptrs.data(), ws.data(), hs.data(), strides.data(), n, threshold, nms_threshold, &spec,
+                                       out_faces_.data(), out_counts_.data(), nullptr, scales_.data() + start, crops.data(), nullptr);
+        if (rc != RF_OK) throw std::runtime_error(string("rf_detect_align_batch: ") + rf_status_string(rc) + ": " + rf_last_error(h_));
+        for (int i = 0; i < n; i++) {
+            const FaceDetectInfo *f = reinterpret_cast<const FaceDetectInfo *>(out_faces_.data() + (size_t)i * opt_.max_faces);
+            last_[start + i].assign(f, f + out_counts_[i]);
+            for (int j = 0; j < std::min(out_counts_[i], opt_.max_crops); j++) {
+                Mat c(opt_.crop_size, opt_.crop_size, CV_8UC3);
+                std::memcpy(c.data, crops.data() + ((size_t)i * opt_.max_crops + j) * crop_bytes, crop_bytes);
+                crops_[start + i].push_back(c);
+            }
         }
     }
 }

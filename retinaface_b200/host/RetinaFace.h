@@ -40,6 +40,8 @@ struct RetinaFaceOptions {
                                          // folding; with net_w = net_h = 0 it also sets the network size.  Empty: built-in graph
     string cache_file;                   // folded-model cache (the reference's "retina.cache", trtnetbase.cpp:205-243, but with a
                                          // staleness check).  Empty: none
+    int crop_size = 112;                 // detectAndAlign: side of the aligned crops (a multiple of 112: the ArcFace template)
+    int max_crops = 16;                  // detectAndAlign: crops of at most this many top-scoring faces per image
 };
 
 class RetinaFace {
@@ -54,6 +56,13 @@ class RetinaFace {
     // compressed input: what main.cpp:18-26 hands to cv::imread.  The JPEG bitstreams are decoded on the GPU
     // (rf_detect_jpeg_batch); results and lastScale() as for detectBatchImages
     void detectEncoded(const vector<vector<unsigned char>> &jpegs, float threshold = 0.5);
+
+    // detection + the step a recognition pipeline takes next (insightface's norm_crop): for each image, crop_size x crop_size
+    // u8 BGR crops of its top max_crops faces, aligned on the GPU by the similarity from their five landmarks to the ArcFace
+    // template and sampled from the ORIGINAL image (rf_detect_align_batch; byte-identical to cv::warpAffine with that matrix).
+    // Faces and lastScale() as for detectBatchImages; crops of image i in lastCrops(i), in score order.
+    void detectAndAlign(vector<cv::Mat> imgs, float threshold = 0.5);
+    const vector<Mat> &lastCrops(size_t i = 0) const { return i < crops_.size() ? crops_[i] : no_crops_; }
 
     // results of the last call, in network-input pixels (RetinaFace.cpp:707); multiply by
     // lastScale() to map back to the caller's image (RetinaFace.cpp:587-591, 732-738)
@@ -79,6 +88,8 @@ class RetinaFace {
     vector<vector<FaceDetectInfo>> last_;
     vector<FaceDetectInfo> empty_;
     vector<float> scales_;
+    vector<vector<Mat>> crops_;
+    vector<Mat> no_crops_;
     vector<rf_face> out_faces_;
     vector<int> out_counts_;
 };

@@ -3,7 +3,9 @@
 // loops forever on a hard-coded JPEG; this one takes a raw BGR image (or synthesises noise) and
 // a finite iteration count so that it can run unattended.
 //   rf_main <model_dir> [--image raw.bgr W H | --jpeg file.jpg] [--net W H] [--iters N] [--batch B] [--thr T] [--tta] [--draw out.bgr]
+//           [--align crops.bgr]
 // --jpeg is the reference's own input form (main.cpp:18: cv::imread of a JPEG): the file's bytes go to the GPU decoder.
+// --align writes the 112 x 112 aligned crops of image 0 (detectAndAlign), one after another, as raw u8 BGR.
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
@@ -25,7 +27,7 @@ int main(int argc, char **argv) {
     opt.net_w = 448; opt.net_h = 448;
     int iters = 1000, batch = 1, iw = 448, ih = 448;
     float thr = 0.9f;
-    string image, draw_path, jpeg;
+    string image, draw_path, jpeg, align_path;
     bool tta = false;
     for (int i = 2; i < argc; i++) {
         if (!strcmp(argv[i], "--image") && i + 3 < argc) { image = argv[i + 1]; iw = atoi(argv[i + 2]); ih = atoi(argv[i + 3]); i += 3; }
@@ -37,6 +39,7 @@ int main(int argc, char **argv) {
         else if (!strcmp(argv[i], "--model") && i + 1 < argc) opt.model_file = argv[++i];
         else if (!strcmp(argv[i], "--tta")) tta = true;
         else if (!strcmp(argv[i], "--draw") && i + 1 < argc) draw_path = argv[++i];
+        else if (!strcmp(argv[i], "--align") && i + 1 < argc) align_path = argv[++i];
     }
     opt.max_batch = batch > opt.max_batch ? batch : opt.max_batch;
     try {
@@ -95,6 +98,13 @@ int main(int argc, char **argv) {
                 std::ofstream o(draw_path, std::ios::binary);
                 for (int y = 0; y < vis.rows; y++) o.write((const char *)vis.data + (size_t)y * vis.step, (std::streamsize)vis.cols * 3);
             }
+        }
+        if (!align_path.empty()) {
+            rf->detectAndAlign(imgs, thr);
+            printf("aligned crops of image 0: %zu (%dx%d u8 BGR) -> %s\n", rf->lastCrops().size(), opt.crop_size, opt.crop_size, align_path.c_str());
+            std::ofstream o(align_path, std::ios::binary);
+            for (const cv::Mat &c : rf->lastCrops())
+                for (int y = 0; y < c.rows; y++) o.write((const char *)c.data + (size_t)y * c.step, (std::streamsize)c.cols * 3);
         }
         delete rf;
     } catch (const std::exception &e) {
